@@ -2,6 +2,7 @@
 """bench.py -- encode_batch throughput of the B200 engine on BASELINE.json's headline config.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mb 1024] [--config gpt2|llama3|wordpiece]
+                    [--dump-outputs DIR]
 
 One step = one pass of the whole hot path (doc_mark -> pretok_scan -> page_scan -> long_find -> bpe_tile -> compaction)
 over one batch of the synthetic corpus of SURVEY.md 8(d) config 2 ("GPT-2 ByteLevel BPE, 1 GB synthetic UTF-8 docs avg
@@ -197,8 +198,39 @@ class DevArr:  # zero-copy torch view of an engine-owned device buffer
         self.__cuda_array_interface__ = {"shape": (count,), "typestr": typestr, "data": (ptr, False), "version": 3}
 
 
-def measure(ctx, cfg, kind, mb, steps, warmup, sharded=False, special=None):
-    """Device-resident and end-to-end numbers of one configuration on this rank.  Returns a dict of raw measurements."""
+DUMP_BYTES = 64 << 20
+DUMP_DOCS = 1 << 15
+
+
+def dump_outputs(out_dir, L, res, n_docs):
+    """Writes what a caller of b2t_encode_batch_device received from one step, as .npy files of at most DUMP_BYTES in all:
+    row_ptr.npy  float64, every stride-th entry of the CSR row pointer (every entry up to 4M documents);
+    docs.npy     float64, a fixed seeded sample of DUMP_DOCS documents (ascending; trimmed to the byte budget);
+    ids.npy      float32, the token ids of those documents, one after the other (exact: ids < 2^24);
+    offsets.npy  float32 [n, 2], their (start, end) char offsets (exact: documents of fewer than 2^24 characters).
+    The same arguments give the same inputs, so two builds can be compared file by file."""
+    import torch
+    T = int(L.b2t_result_n_tokens(res))
+    row_ptr = torch.as_tensor(DevArr(L.b2t_result_row_ptr(res), n_docs + 1, "<i8"), device="cuda").cpu().numpy()
+    stride = max(1, -(-(n_docs + 1) * 8 // (DUMP_BYTES // 2)))
+    docs = np.sort(np.random.default_rng(0).choice(n_docs, size=min(n_docs, DUMP_DOCS), replace=False))
+    lens = row_ptr[docs + 1] - row_ptr[docs]
+    budget = (DUMP_BYTES - row_ptr[::stride].nbytes - docs.nbytes) // 12    # 4 B of id + 8 B of offsets per token
+    docs, lens = docs[np.cumsum(lens) <= budget], lens[np.cumsum(lens) <= budget]
+    tok = np.repeat(row_ptr[docs] - (np.cumsum(lens) - lens), lens) + np.arange(int(lens.sum()))
+    ids, offs = np.zeros(0, np.float32), np.zeros((0, 2), np.float32)
+    if tok.size:
+        idx = torch.from_numpy(tok).cuda()
+        ids = torch.as_tensor(DevArr(L.b2t_result_ids(res), T, "<i4"), device="cuda")[idx].cpu().numpy().astype(np.float32)
+        offs = torch.as_tensor(DevArr(L.b2t_result_offsets(res), 2 * T, "<i4"), device="cuda").view(-1, 2)[idx].cpu().numpy().astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("row_ptr", row_ptr[::stride].astype(np.float64)), ("docs", docs.astype(np.float64)), ("ids", ids), ("offsets", offs)):
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
+def measure(ctx, cfg, kind, mb, steps, warmup, sharded=False, special=None, dump=None):
+    """Device-resident and end-to-end numbers of one configuration on this rank.  Returns a dict of raw measurements.
+    dump: a directory that receives what the last timed device-resident step computed (dump_outputs)."""
     import torch
     from tokenizers_b200 import Tokenizer, _lib
     L, rank, world, local = ctx["L"], ctx["rank"], ctx["world"], ctx["local"]
@@ -226,10 +258,12 @@ def measure(ctx, cfg, kind, mb, steps, warmup, sharded=False, special=None):
     stream = torch.cuda.current_stream()
     _lib.check(L.b2t_engine_set_profiling(tok.handle, 1))
 
-    def step_device():
+    def step_device(keep=False):
         res = ctypes.c_void_p()
         _lib.check(L.b2t_encode_batch_device(tok.handle, d_bytes.data_ptr(), n, d_off.data_ptr(), n_docs, flags, ctypes.c_void_p(stream.cuda_stream), ctypes.byref(res)))
         T = L.b2t_result_n_tokens(res)
+        if keep:   # the result stays valid until the next call on the engine or b2t_result_free
+            return T, res
         L.b2t_result_free(res)
         return T
 
@@ -245,8 +279,11 @@ def measure(ctx, cfg, kind, mb, steps, warmup, sharded=False, special=None):
     kern_ms, launches = {}, 0
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(stream)
-    for _ in range(steps):
-        T = step_device()
+    for i in range(steps):
+        if dump and i == steps - 1:
+            T, kept = step_device(keep=True)
+        else:
+            T = step_device()
         launches += L.b2t_engine_last_kernels(tok.handle, names, ms, 16)
         for i in range(16):
             if names[i] is None:
@@ -257,6 +294,10 @@ def measure(ctx, cfg, kind, mb, steps, warmup, sharded=False, special=None):
     ev1.record(stream)
     barrier()
     dev_ms = ev0.elapsed_time(ev1)
+    if dump:
+        if rank == 0:
+            dump_outputs(dump, L, kept, n_docs)
+        L.b2t_result_free(kept)
     _lib.check(L.b2t_engine_set_profiling(tok.handle, 0))
 
     # ---- N > 1: the sharded product path, exchange of step i overlapping the kernels of step i + 1
@@ -397,7 +438,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the secondary configs (llama3 / wordpiece / skew)")
     ap.add_argument("--kind", type=int, default=0, help="corpus kind override (5 = length-skew stress of BASELINE configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed device-resident step computed to DIR/<name>.npy "
+                    "(rank 0's batch; a seeded sample, at most 64 MiB: see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3) if a.impl != "reference" else a.warmup
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     cfg = a.config
@@ -441,7 +486,7 @@ def main():
     if rank == 0:
         sampler.start()  # samples every 50 ms from the warm-up through the timed device and e2e regions
     kind = a.kind or KIND[cfg]
-    m = measure(ctx, cfg, kind, a.mb, a.steps, a.warmup, sharded=True)
+    m = measure(ctx, cfg, kind, a.mb, a.steps, a.warmup, sharded=True, dump=a.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- reduce over ranks: time = max, work = sum

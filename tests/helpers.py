@@ -1,5 +1,5 @@
 """Shared test helpers (golden loading, CSR flattening, wheel access)."""
-import gzip, json, os
+import gzip, hashlib, json, os
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -87,6 +87,64 @@ def wheel():
 def wheel_csr(tok, docs):
     encs = tok.encode_batch(docs, add_special_tokens=False)
     return cases_to_csr([{"ids": e.ids, "offsets": e.offsets, "word_ids": e.word_ids} for e in encs])
+
+
+# ---------------------------------------------------------------------------------------------- recorded reference outputs
+# What the reference implementation (the `tokenizers` wheel) returned for the tests' seeded inputs, kept as truncated SHA-256
+# digests of a canonical JSON form, so that every comparison with it runs without the wheel and the file stays small.
+# To record them again (the wheel importable): B2T_RECORD_REFERENCE=1 python -m pytest tests -k <tests>.  Every
+# reference() call then runs the wheel and rewrites its entry.  The GPU tests record before they create the engine, so a
+# machine without a GPU records their entries too (and then fails their engine part).
+REFERENCE_DIGESTS = os.path.join(GOLDEN, "reference_digests.json")
+RECORDING = os.environ.get("B2T_RECORD_REFERENCE") == "1"
+_digests = None
+
+
+def _plain(x):
+    if isinstance(x, np.ndarray):
+        return x.tolist()
+    if isinstance(x, np.generic):
+        return x.item()
+    if isinstance(x, dict):
+        return {str(k): _plain(v) for k, v in x.items()}
+    if isinstance(x, (list, tuple)):
+        return [_plain(v) for v in x]
+    return x
+
+
+def digest(x):
+    js = json.dumps(_plain(x), sort_keys=True, separators=(",", ":"), ensure_ascii=False)
+    return hashlib.sha256(js.encode("utf-8")).hexdigest()[:16]
+
+
+def csr_plain(csr):
+    """(ids, offsets, word_ids, row_ptr) in the form assert_csr_equal compares: flat, whatever the integer type"""
+    return [np.asarray(a).reshape(-1).astype(np.int64) for a in csr]
+
+
+def reference(key, fn):
+    """The recorded digest of what the reference returned for `key`; when recording, fn() runs the wheel and replaces it."""
+    global _digests
+    if _digests is None:
+        _digests = json.load(open(REFERENCE_DIGESTS))["digests"] if os.path.exists(REFERENCE_DIGESTS) else {}
+    if RECORDING:
+        _digests[key] = digest(fn())
+        with open(REFERENCE_DIGESTS, "w") as f:
+            json.dump({"generator": "B2T_RECORD_REFERENCE=1 python -m pytest tests (see tests/helpers.py)",
+                       "tokenizers": wheel().__version__, "digests": dict(sorted(_digests.items()))}, f, indent=0)
+            f.write("\n")
+    assert key in _digests, f"no recorded reference output for {key}"
+    return _digests[key]
+
+
+def assert_reference(key, got, fn, what=""):
+    """got must equal what the reference returned for `key` (fn() computes that with the wheel, only when recording)"""
+    assert digest(got) == reference(key, fn), f"{what or key}: differs from the reference implementation's recorded output ({key})"
+
+
+def wheel_tokenizer(tokenizer_json):
+    """the reference's Tokenizer when recording, else None (the tests then compare with the recorded digests only)"""
+    return wheel().Tokenizer.from_str(tokenizer_json) if RECORDING else None
 
 
 # ---------------------------------------------------------------------------------------------- host-logic harness

@@ -1,10 +1,10 @@
 """Host steps either side of the hot path: added-token extraction (added_vocabulary.rs:430-564) and the single-sequence
 special-token template (processors/template.rs).  CPU: tokenizers_b200's host logic in front of the oracle, against the
-reference wheel (when importable) and against committed golden vectors.  GPU: the same through the real engine."""
-import gzip, json, os
+reference wheel's recorded outputs and against committed golden vectors.  GPU: the same through the real engine."""
+import gzip, json, os, types
 import numpy as np
 import pytest
-from helpers import GOLDEN, asset_json, with_added_tokens, added_token_docs, oracle_backed_tokenizer, wheel
+from helpers import GOLDEN, asset_json, with_added_tokens, added_token_docs, oracle_backed_tokenizer, assert_reference, wheel, wheel_tokenizer
 
 CONFIGS = [("gpt2_style", False), ("gpt2_style", True), ("llama3_style", False), ("wordpiece", True)]
 
@@ -30,36 +30,33 @@ def _compare(got, exp, docs, what):
 @pytest.mark.parametrize("asset,template", CONFIGS)
 @pytest.mark.parametrize("prefix_space", [False, True])
 def test_host_logic_vs_wheel(asset, template, prefix_space):
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
     if prefix_space and asset != "gpt2_style":
         pytest.skip("add_prefix_space only varies for the ByteLevel pre-tokenizer")
     tj = with_added_tokens(_patched(asset, prefix_space), template)
-    ref = tk.Tokenizer.from_str(tj)
+    ref = wheel_tokenizer(tj)
     mine = oracle_backed_tokenizer(tj)
     docs = added_token_docs(7, 1500)
+    assert_reference("added/docs/7_1500", docs, lambda: docs)
+    key = f"added/host_logic/{asset}/template={template}/prefix_space={prefix_space}"
     for special in (False, True):
-        exp = _flat(ref.encode_batch(docs, add_special_tokens=special))
-        got = _flat(mine.encode_batch(docs, add_special_tokens=special))
-        _compare(got, exp, docs, f"{asset} template={template} add_special_tokens={special}")
-    assert mine.token_to_id("<mask>") == ref.token_to_id("<mask>")
+        assert_reference(f"{key}/special={special}", _flat(mine.encode_batch(docs, add_special_tokens=special)),
+                         lambda: _flat(ref.encode_batch(docs, add_special_tokens=special)), f"{asset} template={template} add_special_tokens={special}")
+    assert_reference(f"{key}/mask_id", mine.token_to_id("<mask>"), lambda: ref.token_to_id("<mask>"))
     assert mine.id_to_token(mine.token_to_id("<a><b>")) == "<a><b>"
-    assert mine.get_vocab_size() == ref.get_vocab_size() and mine.get_vocab_size(False) == ref.get_vocab_size(False)
+    assert_reference(f"{key}/vocab_size", [mine.get_vocab_size(), mine.get_vocab_size(False)], lambda: [ref.get_vocab_size(), ref.get_vocab_size(False)])
 
 
 def test_byte_offsets_and_fast_vs_wheel():
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
     tj = with_added_tokens(asset_json("gpt2_style"), True)
     mine = oracle_backed_tokenizer(tj)
     docs = added_token_docs(11, 400)
+    assert_reference("added/docs/11_400", docs, lambda: docs)
     full = mine.encode_batch(docs, add_special_tokens=True)
     fast = mine.encode_batch_fast(docs, add_special_tokens=True)
     assert [e.ids for e in full] == [e.ids for e in fast]
     # (token texts are not compared: without offsets the reference reports '' for added tokens found in the text)
-    _compare(_flat(fast, False), _flat(tk.Tokenizer.from_str(tj).encode_batch_fast(docs, add_special_tokens=True), False), docs, "encode_batch_fast")
+    assert_reference("added/encode_batch_fast", _flat(fast, False), lambda: _flat(wheel_tokenizer(tj).encode_batch_fast(docs, add_special_tokens=True), False),
+                     "encode_batch_fast")
     # byte offsets of the CSR entry point == char offsets mapped through the document's UTF-8 encoding
     data = np.frombuffer("".join(docs).encode("utf-8"), dtype=np.uint8)
     off = np.zeros(len(docs) + 1, dtype=np.uint64)
@@ -90,18 +87,17 @@ def _post_processors(js):
 @pytest.mark.parametrize("asset,prefix_space", [("gpt2_style", False), ("gpt2_style", True), ("llama3_style", None)])
 def test_post_processors_vs_wheel(asset, prefix_space):
     """offset trimming (byte_level.rs:202-234) and the Bert / Roberta / Template / Sequence processors for single sequences"""
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
     base = json.loads(with_added_tokens(_patched(asset, prefix_space)))
     docs = added_token_docs(13, 300) + ["  two  spaces  ", " x", "x ", "   ", " <mask> y", "a  <both>  b"]
-    for pp in _post_processors(base):
+    assert_reference("added/docs/13_300", docs, lambda: docs)
+    for i, pp in enumerate(_post_processors(base)):
         js = dict(base, post_processor=pp)
         tj = json.dumps(js)
-        ref, mine = tk.Tokenizer.from_str(tj), oracle_backed_tokenizer(tj)
+        ref, mine = wheel_tokenizer(tj), oracle_backed_tokenizer(tj)
         for special in (False, True):
-            _compare(_flat(mine.encode_batch(docs, add_special_tokens=special)), _flat(ref.encode_batch(docs, add_special_tokens=special)),
-                     docs, f"{asset} {pp['type']} trim={pp.get('trim_offsets')} aps={pp.get('add_prefix_space')} special={special}")
+            assert_reference(f"added/post_processors/{asset}/prefix_space={prefix_space}/{i}/special={special}",
+                             _flat(mine.encode_batch(docs, add_special_tokens=special)), lambda: _flat(ref.encode_batch(docs, add_special_tokens=special)),
+                             f"{asset} {pp['type']} trim={pp.get('trim_offsets')} aps={pp.get('add_prefix_space')} special={special}")
 
 
 def test_candidate_start_inside_a_run_across_documents():
@@ -115,10 +111,8 @@ def test_candidate_start_inside_a_run_across_documents():
     encs = mine.encode_batch(["a ", "  x>", "b", "   "], add_special_tokens=False)
     assert encs[1].ids[0] == tid and encs[1].offsets[0] == (0, 2)
     assert encs[3].ids[0] == tid and encs[3].offsets[:2] == [(0, 2), (2, 3)]
-    tk = wheel()
-    if tk is not None:
-        ref = tk.Tokenizer.from_str(json.dumps(js)).encode_batch(["a ", "  x>", "b", "   "], add_special_tokens=False)
-        _compare(_flat(encs), _flat(ref), ["a ", "  x>", "b", "   "], "boundary run")
+    assert_reference("added/boundary_run", _flat(encs),
+                     lambda: _flat(wheel_tokenizer(json.dumps(js)).encode_batch(["a ", "  x>", "b", "   "], add_special_tokens=False)), "boundary run")
 
 
 def _flat_full(encs):
@@ -132,37 +126,37 @@ def _flat_full(encs):
 @pytest.mark.parametrize("asset,template", [("gpt2_style", True), ("wordpiece", False)])
 def test_truncation_and_padding_vs_wheel(asset, template):
     """TokenizerImpl::post_process steps 1 and 3 (utils/truncation.rs, Encoding::truncate, utils/padding.rs) for single sequences"""
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
     tj = with_added_tokens(asset_json(asset), template)
-    ref, mine = tk.Tokenizer.from_str(tj), oracle_backed_tokenizer(tj)
+    ref, mine = wheel_tokenizer(tj), oracle_backed_tokenizer(tj)
     docs = added_token_docs(17, 150) + ["", "a", "a b c d e f g h i j k l m n o p q r s t u v w x y z " * 3]
+    assert_reference("added/docs/17_150", docs, lambda: docs)
+    key = f"added/truncation/{asset}/template={template}"
     cases = [dict(max_length=8, stride=0, direction="right"), dict(max_length=8, stride=3, direction="right"),
              dict(max_length=7, stride=2, direction="left"), dict(max_length=3, stride=0, direction="left"),
              dict(max_length=16, stride=5, direction="right", strategy="only_first")]
     pads = [None, dict(direction="left", pad_id=3, pad_type_id=1, pad_token="<pad>"), dict(length=12), dict(pad_to_multiple_of=8)]
     for ci, tc in enumerate(cases):
         for pi, pc in enumerate(pads):
-            for t in (ref, mine):
+            for t in filter(None, (ref, mine)):
                 t.enable_truncation(**tc)
                 t.no_padding() if pc is None else t.enable_padding(**pc)
             for special in (False, True):
-                exp = _flat_full(ref.encode_batch(docs, add_special_tokens=special))
-                got = _flat_full(mine.encode_batch(docs, add_special_tokens=special))
-                _compare(got, exp, docs, f"{asset} trunc={tc} pad={pc} special={special}")
+                assert_reference(f"{key}/{ci}/{pi}/special={special}", _flat_full(mine.encode_batch(docs, add_special_tokens=special)),
+                                 lambda: _flat_full(ref.encode_batch(docs, add_special_tokens=special)), f"{asset} trunc={tc} pad={pc} special={special}")
     # padding without truncation, settings read from tokenizer.json
     js = json.loads(tj)
     js["truncation"] = {"direction": "Right", "max_length": 10, "strategy": "LongestFirst", "stride": 2}
     js["padding"] = {"strategy": {"Fixed": 14}, "direction": "Right", "pad_to_multiple_of": None, "pad_id": 1, "pad_type_id": 0, "pad_token": "[PAD]"}
-    ref, mine = tk.Tokenizer.from_str(json.dumps(js)), oracle_backed_tokenizer(json.dumps(js))
-    assert mine.truncation == ref.truncation and mine.padding["length"] == 14
-    _compare(_flat_full(mine.encode_batch(docs)), _flat_full(ref.encode_batch(docs)), docs, "settings from tokenizer.json")
+    ref, mine = wheel_tokenizer(json.dumps(js)), oracle_backed_tokenizer(json.dumps(js))
+    assert_reference(f"{key}/json_settings", mine.truncation, lambda: ref.truncation)
+    assert mine.padding["length"] == 14
+    assert_reference(f"{key}/json_settings/encodings", _flat_full(mine.encode_batch(docs)), lambda: _flat_full(ref.encode_batch(docs)), "settings from tokenizer.json")
     def toks(encs):  # the text of an lstrip / rstrip token is its matched span (Token::new(id, value, ..), added_vocabulary.rs:508)
         return [(e.tokens, [o.tokens for o in e.overflowing]) for e in encs]
-    assert toks(mine.encode_batch(docs)) == toks(ref.encode_batch(docs))
-    ref.no_truncation(); mine.no_truncation()
-    _compare(_flat_full(mine.encode_batch(docs)), _flat_full(ref.encode_batch(docs)), docs, "padding only")
+    assert_reference(f"{key}/json_settings/tokens", toks(mine.encode_batch(docs)), lambda: toks(ref.encode_batch(docs)))
+    for t in filter(None, (ref, mine)):
+        t.no_truncation()
+    assert_reference(f"{key}/padding_only", _flat_full(mine.encode_batch(docs)), lambda: _flat_full(ref.encode_batch(docs)), "padding only")
 
 
 def test_unsupported_post_processors():
@@ -274,26 +268,25 @@ def test_gpu_decreasing_doc_off_is_rejected():
 def test_pretokenized_input_vs_wheel(asset):
     """is_pretokenized=True (tokenizer/mod.rs:762-805): words are encoded one by one, offsets stay relative to the word,
     word ids are the word's index -- with added tokens, a template, truncation and padding on top"""
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
     import random
     from fuzzgen import rand_doc
     rng = random.Random(3)
     tj = with_added_tokens(_patched(asset, True if asset == "gpt2_style" else None), True)
-    ref, mine = tk.Tokenizer.from_str(tj), oracle_backed_tokenizer(tj)
+    ref, mine = wheel_tokenizer(tj), oracle_backed_tokenizer(tj)
     pool = ["hello", "world", "don't", "<mask>", " x", "", "a<|endoftext|>b", "tok", "Zürich", "  ", "multi word item", "日本語", "1234567", "wörd"]
     seqs = [[]] + [[rng.choice(pool) if rng.random() < 0.6 else rand_doc(rng, 5) for _ in range(rng.randint(0, 9))] for _ in range(300)]
+    assert_reference("added/docs/pretokenized", seqs, lambda: seqs)
+    key = f"added/pretokenized/{asset}"
     for special in (False, True):
-        _compare(_flat(mine.encode_batch(seqs, is_pretokenized=True, add_special_tokens=special)),
-                 _flat(ref.encode_batch(seqs, is_pretokenized=True, add_special_tokens=special)), seqs, f"{asset} pretokenized special={special}")
-    for t in (ref, mine):
+        assert_reference(f"{key}/special={special}", _flat(mine.encode_batch(seqs, is_pretokenized=True, add_special_tokens=special)),
+                         lambda: _flat(ref.encode_batch(seqs, is_pretokenized=True, add_special_tokens=special)), f"{asset} pretokenized special={special}")
+    for t in filter(None, (ref, mine)):
         t.enable_truncation(max_length=6, stride=2)
         t.enable_padding(pad_to_multiple_of=4)
-    _compare(_flat_full(mine.encode_batch(seqs, is_pretokenized=True)), _flat_full(ref.encode_batch(seqs, is_pretokenized=True)), seqs,
-             f"{asset} pretokenized + truncation + padding")
+    assert_reference(f"{key}/truncation_padding", _flat_full(mine.encode_batch(seqs, is_pretokenized=True)),
+                     lambda: _flat_full(ref.encode_batch(seqs, is_pretokenized=True)), f"{asset} pretokenized + truncation + padding")
     e = mine.encode(["hello", "world"], is_pretokenized=True)
-    assert e.ids == list(ref.encode(["hello", "world"], is_pretokenized=True).ids)
+    assert_reference(f"{key}/hello_world", list(e.ids), lambda: list(ref.encode(["hello", "world"], is_pretokenized=True).ids))
     with pytest.raises(TypeError):
         mine.encode_batch(["not a list of words"], is_pretokenized=True)
 
@@ -315,9 +308,6 @@ def _pair_processors(js):
 def test_pairs_vs_wheel():
     """EncodeInput::Dual: both sequences through the engine, then truncation strategies, the pair templates and the merge
     with every combination of overflowing parts (pairs.py), padding -- against the reference, mixed with single inputs"""
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
     import random
     rng = random.Random(8)
     base = json.loads(with_added_tokens(_patched("gpt2_style", True)))
@@ -325,68 +315,76 @@ def test_pairs_vs_wheel():
     inputs = [(rng.choice(texts), rng.choice(texts)) if rng.random() < 0.7 else rng.choice(texts) for _ in range(45)] + [("", ""), ("a", ""), ("", "b")]
     truncs = [None, dict(max_length=12, stride=0), dict(max_length=9, stride=2, direction="left"), dict(max_length=11, stride=3, strategy="only_first"),
               dict(max_length=14, stride=1, strategy="only_second"), dict(max_length=7, stride=1, strategy="longest_first")]
+    assert_reference("added/docs/pairs", inputs, lambda: inputs)
+
+    def refused(tok, special, error):
+        """indices of the inputs the tokenizer refuses (one by one only when the whole batch is refused)"""
+        try:
+            tok.encode_batch(inputs, add_special_tokens=special)
+            return []
+        except error:
+            out = []
+            for i, x in enumerate(inputs):
+                try:
+                    tok.encode(*((x,) if isinstance(x, str) else x), add_special_tokens=special)
+                except error:
+                    out.append(i)
+            return out
     for pi, pp in enumerate(_pair_processors(base)):
         tj = json.dumps(dict(base, post_processor=pp))
-        ref, mine = tk.Tokenizer.from_str(tj), oracle_backed_tokenizer(tj)
+        ref, mine = wheel_tokenizer(tj), oracle_backed_tokenizer(tj)
         for ti, tc in enumerate(truncs):
-            for t in (ref, mine):
+            for t in filter(None, (ref, mine)):
                 t.no_truncation() if tc is None else t.enable_truncation(**tc)
                 t.enable_padding(pad_to_multiple_of=4) if (ti + pi) % 3 == 0 else t.no_padding()
             for special in (False, True):
                 # some (input, setting) combinations are errors in the reference (a strategy that cannot shorten the input
                 # enough, a stride that no longer fits once the special tokens are subtracted): they must be errors here too
-                batch = inputs
-                try:
-                    exp = _flat_full(ref.encode_batch(batch, add_special_tokens=special))
-                except BaseException:
-                    batch = []
-                    for x in inputs:
-                        args = (x,) if isinstance(x, str) else x
-                        try:
-                            ref.encode(*args, add_special_tokens=special)
-                            batch.append(x)
-                        except BaseException:
-                            with pytest.raises(ValueError):
-                                mine.encode(*args, add_special_tokens=special)
-                    exp = _flat_full(ref.encode_batch(batch, add_special_tokens=special))
-                got = _flat_full(mine.encode_batch(batch, add_special_tokens=special))
-                _compare(got, exp, batch, f"pairs pp={pp and pp['type']} trunc={tc} special={special}")
-        for t in (ref, mine):
+                key, what = f"added/pairs/{pi}/{ti}/special={special}", f"pairs pp={pp and pp['type']} trunc={tc} special={special}"
+                bad = refused(mine, special, ValueError)
+                assert_reference(f"{key}/refused", bad, lambda: refused(ref, special, BaseException), what)
+                batch = [x for i, x in enumerate(inputs) if i not in bad]
+                assert_reference(key, _flat_full(mine.encode_batch(batch, add_special_tokens=special)),
+                                 lambda: _flat_full(ref.encode_batch(batch, add_special_tokens=special)), what)
+        for t in filter(None, (ref, mine)):
             t.no_truncation(); t.no_padding()
-        e_ref, e_mine = ref.encode("hello world", "x <mask> y"), mine.encode("hello world", "x <mask> y")
-        assert e_mine.sequence_ids == e_ref.sequence_ids and e_mine.n_sequences == e_ref.n_sequences and e_mine.type_ids == e_ref.type_ids
+
+        def seqs(e):
+            return [e.sequence_ids, e.n_sequences, e.type_ids]
+        assert_reference(f"added/pairs/{pi}/sequence_ids", seqs(mine.encode("hello world", "x <mask> y")), lambda: seqs(ref.encode("hello world", "x <mask> y")))
 
 
 def test_decode_vs_wheel():
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
-    for asset, dec in (("gpt2_style", {"type": "ByteLevel", "add_prefix_space": True, "trim_offsets": True, "use_regex": True}),
-                       ("wordpiece", {"type": "WordPiece", "prefix": "##", "cleanup": True}), ("wordpiece", None)):
+    for i, (asset, dec) in enumerate((("gpt2_style", {"type": "ByteLevel", "add_prefix_space": True, "trim_offsets": True, "use_regex": True}),
+                                      ("wordpiece", {"type": "WordPiece", "prefix": "##", "cleanup": True}), ("wordpiece", None))):
         js = json.loads(with_added_tokens(asset_json(asset), True))
         js["decoder"] = dec
         tj = json.dumps(js)
-        ref, mine = tk.Tokenizer.from_str(tj), oracle_backed_tokenizer(tj)
+        ref, mine = wheel_tokenizer(tj), oracle_backed_tokenizer(tj)
         docs = added_token_docs(5, 300) + ["I do not know , it 's fine . don't you ?"]
-        encs = ref.encode_batch(docs)
+        ids = [list(e.ids) for e in mine.encode_batch(docs)]
+        assert_reference(f"added/decode/{i}/ids", ids, lambda: [e.ids for e in ref.encode_batch(docs)])
         for skip in (True, False):
-            assert mine.decode_batch([e.ids for e in encs], skip_special_tokens=skip) == ref.decode_batch([e.ids for e in encs], skip_special_tokens=skip)
-        assert mine.decode([10 ** 9, 5]) == ref.decode([10 ** 9, 5])  # unknown ids are dropped
+            assert_reference(f"added/decode/{i}/skip={skip}", mine.decode_batch(ids, skip_special_tokens=skip), lambda: ref.decode_batch(ids, skip_special_tokens=skip))
+        assert_reference(f"added/decode/{i}/unknown", mine.decode([10 ** 9, 5]), lambda: ref.decode([10 ** 9, 5]))  # unknown ids are dropped
 
 
 def test_add_tokens_vs_wheel():
     """Tokenizer.add_tokens / add_special_tokens after loading: id assignment and extraction follow the reference"""
-    tk = wheel()
-    if tk is None:
-        pytest.skip("reference wheel not importable")
     tj = asset_json("gpt2_style")
-    ref, mine = tk.Tokenizer.from_str(tj), oracle_backed_tokenizer(tj)
-    at = tk.AddedToken
-    for t in (ref, mine):
+    ref, mine = wheel_tokenizer(tj), oracle_backed_tokenizer(tj)
+
+    def at(t, content, **kw):   # the reference's AddedToken(content, **kw), or what it carries for a token that is not special
+        if t is ref:
+            return wheel().AddedToken(content, **kw)
+        return types.SimpleNamespace(**dict(dict(content=content, single_word=False, lstrip=False, rstrip=False, normalized=True), **kw))
+    for t in filter(None, (ref, mine)):
         assert t.add_special_tokens(["<|endoftext|>", "<pad>"]) == 2
-        assert t.add_tokens(["hello", "newword", at("tok", single_word=True), at("<x>", lstrip=True, rstrip=True)]) == 4
+        assert t.add_tokens(["hello", "newword", at(t, "tok", single_word=True), at(t, "<x>", lstrip=True, rstrip=True)]) == 4
         assert t.add_tokens(["newword"]) == 0
-    assert mine.get_vocab_size() == ref.get_vocab_size() and mine.get_vocab() == ref.get_vocab()
-    assert mine.num_special_tokens_to_add(False) == ref.num_special_tokens_to_add(False) == 0
+    assert_reference("added/add_tokens/vocab", [mine.get_vocab_size(), mine.get_vocab()], lambda: [ref.get_vocab_size(), ref.get_vocab()])
+    assert mine.num_special_tokens_to_add(False) == 0
+    assert_reference("added/add_tokens/num_special_tokens_to_add", mine.num_special_tokens_to_add(False), lambda: ref.num_special_tokens_to_add(False))
     docs = ["hello newword <|endoftext|> x  <x>  y tok atok <pad>", "newwordnewword", ""] + added_token_docs(4, 200)
-    _compare(_flat(mine.encode_batch(docs)), _flat(ref.encode_batch(docs)), docs, "after add_tokens")
+    assert_reference("added/docs/4_200", docs, lambda: docs)
+    assert_reference("added/add_tokens/encodings", _flat(mine.encode_batch(docs)), lambda: _flat(ref.encode_batch(docs)), "after add_tokens")

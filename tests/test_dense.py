@@ -1,12 +1,10 @@
 """Dense mode (b2t_encode_batch_dense*): special-token template + truncation + padding on the device.
-CPU: the oracle-side restatement (oracle.dense_rows) against the reference wheel.  GPU: the engine against both."""
+CPU: the oracle-side restatement (oracle.dense_rows) against the reference wheel's recorded outputs.  GPU: the engine against both."""
 import ctypes, json, os
 import numpy as np
 import pytest
 import helpers, fuzzgen, corpus
 from oracle import oracle as orc
-
-tk = helpers.wheel()
 
 TEMPLATES = {
     "gpt2_style": lambda v: {"type": "TemplateProcessing",
@@ -50,7 +48,7 @@ def spec_of(js, tr, pd):
 
 
 def wheel_dense(js, docs, tr, pd):
-    tok = tk.Tokenizer.from_str(js)
+    tok = helpers.wheel_tokenizer(js)
     if tr:
         tok.enable_truncation(tr["max_length"], direction=tr["direction"])
     tok.enable_padding(direction=pd["direction"], pad_id=pd["pad_id"], length=pd["length"], pad_to_multiple_of=pd.get("pad_to_multiple_of"))
@@ -59,18 +57,17 @@ def wheel_dense(js, docs, tr, pd):
             np.array([e.attention_mask for e in encs], dtype=np.uint8).reshape(len(docs), -1))
 
 
-@pytest.mark.skipif(tk is None, reason="reference wheel not importable")
 @pytest.mark.parametrize("name", list(TEMPLATES))
 def test_oracle_dense_matches_wheel(name):
     js = tokenizer_json(name)
     o = orc.Oracle(js)
     docs = docs_for(11)
+    helpers.assert_reference("dense/docs11", docs, lambda: docs)
     ids, _, _, rp = o.encode_batch(docs)
-    for tr, pd in SETTINGS:
+    for k, (tr, pd) in enumerate(SETTINGS):
         got = orc.dense_rows(ids, rp, **spec_of(js, tr, pd))
-        exp = wheel_dense(js, docs, tr, pd)
-        assert np.array_equal(got[0], exp[0]) and np.array_equal(got[1], exp[1]), (name, tr, pd)
-        assert np.array_equal(got[2], exp[1].sum(axis=1))
+        helpers.assert_reference(f"dense/{name}/{k}/docs11", got[:2], lambda: wheel_dense(js, docs, tr, pd), f"{name} {tr} {pd}")
+        assert np.array_equal(got[2], got[1].sum(axis=1))
 
 
 def _golden():
@@ -102,18 +99,19 @@ def _apply(tok, tr, pd):
 def test_gpu_dense_matches_oracle_and_wheel(name):
     from tokenizers_b200 import Tokenizer
     js = tokenizer_json(name)
-    tok, o = Tokenizer.from_str(js), orc.Oracle(js)
     docs = docs_for(12)
+    helpers.assert_reference("dense/docs12", docs, lambda: docs)
+    # the reference's outputs first, so that recording them needs no GPU
+    wheel = [helpers.reference(f"dense/{name}/{k}/docs12", lambda: wheel_dense(js, docs, tr, pd)) for k, (tr, pd) in enumerate(SETTINGS)]
+    tok, o = Tokenizer.from_str(js), orc.Oracle(js)
     ids, _, _, rp = o.encode_batch(docs)
-    for tr, pd in SETTINGS:
+    for k, (tr, pd) in enumerate(SETTINGS):
         _apply(tok, tr, pd)
         got = tok.encode_batch_dense(docs)
         exp = orc.dense_rows(ids, rp, **spec_of(js, tr, pd))
         assert got["input_ids"].shape == exp[0].shape, (name, tr, pd)
         assert np.array_equal(got["input_ids"], exp[0]) and np.array_equal(got["attention_mask"], exp[1]) and np.array_equal(got["lengths"], exp[2]), (name, tr, pd)
-        if tk is not None:
-            w = wheel_dense(js, docs, tr, pd)
-            assert np.array_equal(got["input_ids"], w[0]) and np.array_equal(got["attention_mask"], w[1]), (name, tr, pd, "wheel")
+        assert helpers.digest((got["input_ids"], got["attention_mask"])) == wheel[k], (name, tr, pd, "wheel")
     g = _golden()   # and the committed vectors of the wheel
     for k, (tr, pd) in enumerate(SETTINGS):
         _apply(tok, tr, pd)

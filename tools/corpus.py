@@ -1,5 +1,5 @@
 """ctypes wrapper over tools/corpus_gen.c (synthetic corpora of SURVEY.md §8(d)).  Test/bench infrastructure."""
-import ctypes, os, subprocess
+import ctypes, os, subprocess, tempfile
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -8,8 +8,12 @@ _SRC = os.path.join(_HERE, "corpus_gen.c")
 
 
 def build(force=False):
+    """Path of the generator library, compiled when missing or older than its source (into a temporary directory when
+    the tree is read-only)."""
     if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(_SRC):
-        subprocess.check_call(["gcc", "-O2", "-shared", "-fPIC", "-o", _SO, _SRC, "-lm"])
+        so = _SO if os.access(_HERE, os.W_OK) else os.path.join(tempfile.mkdtemp(prefix="b2t_corpus_"), "libcorpus.so")
+        subprocess.check_call(["gcc", "-O2", "-shared", "-fPIC", "-o", so, _SRC, "-lm"])
+        return so
     return _SO
 
 
